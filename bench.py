@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: correspondence-sets/sec through PointDSC.forward (testing mode).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one testing-mode forward over one batch of B synthetic correspondence sets (default: the configuration
@@ -63,7 +63,14 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip bs=1 latency / config-D sweep / strong scaling")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (final_trans, final_labels) as DIR/<name>.npy, float32")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "engine":
+        ap.error("--dump-outputs writes the engine's outputs: use it with --impl engine")
+    return a
 
 
 def config_of(args, world):
@@ -319,6 +326,27 @@ def time_steps(model, d, steps, keep=False):
     return e0.elapsed_time(e1), outs
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, out, rank, world):
+    """`out` (what one step returned) as <directory>/<name>.npy, with a _rank<r> suffix when several ranks write.  Outputs over
+    64 MB in all are cut to a seeded sample of the sets, whose indices in the batch are written as sets.npy."""
+    import numpy as np
+    arrays = {k: v.cpu().numpy() for k, v in out.items()}
+    B = len(arrays["final_trans"])
+    per_set = sum(a[0].nbytes for a in arrays.values())
+    budget = DUMP_BYTES // world - 4096                 # this rank's share, less the .npy headers
+    if B * per_set > budget:
+        keep = np.sort(np.random.default_rng(0).choice(B, budget // (per_set + 8), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["sets"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}{suffix}.npy"), a)
+
+
 def run_engine(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -378,6 +406,8 @@ def run_engine(args, rank, world, local_rank):
     identical = all(torch.equal(o["final_trans"], outs[0]["final_trans"]) and torch.equal(o["final_labels"], outs[0]["final_labels"])
                     for o in outs[1:])
     assert identical, "outputs of the timed steps differ although their inputs are identical"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, rank, world)
 
     # sanity: the timed work produced registrations (not a skipped / cached forward)
     err = (out["final_trans"].cpu() - host["gt_trans"]).abs().amax(dim=(1, 2))

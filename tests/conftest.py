@@ -1,6 +1,7 @@
 import glob
 import json
 import os
+import re
 import sys
 
 import numpy as np
@@ -42,6 +43,24 @@ def load_case(path):
     case = {k: z[k] for k in z.files if k != "meta"}
     case["meta"] = json.loads(str(z["meta"]))
     return case
+
+
+def demo_clouds(directory):
+    """The reference's demo clouds shrunk to one vertex per 5 cm voxel (tests/golden/make_demo_clouds_golden.py), written under
+    `directory` as cloud_bin_{0,1}.ply behind the files' own headers.  Returns (paths, vertex counts of the full clouds, the
+    vertices written)."""
+    z = np.load(os.path.join(GOLDEN, "demo_clouds_sample.npz"))
+    paths, counts, points = [], [], []
+    for i in (0, 1):
+        head, pts = bytes(z[f"header_{i}"]).decode("ascii"), z[f"points_{i}"]
+        full = re.search(r"^element vertex (\d+)$", head, re.M)
+        counts.append(int(full.group(1)))
+        paths.append(os.path.join(str(directory), f"cloud_bin_{i}.ply"))
+        with open(paths[-1], "wb") as f:
+            f.write((head[:full.start(1)] + str(len(pts)) + head[full.end(1):]).encode("ascii"))
+            f.write(pts.astype("<f4").tobytes())
+        points.append(pts)
+    return paths, counts, points
 
 
 def registration_ok(case):

@@ -138,3 +138,48 @@ def test_bench_reference_arm_contract():
     assert d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"] == {"value": d["value"], "unit": "sets/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"]
+
+
+def test_bench_dump_outputs_names_and_size_cap(tmp_path):
+    """`bench.py --dump-outputs`: one float32 .npy per returned array; above 64 MB a seeded sample of the sets, the same one
+    every run, with its indices."""
+    import numpy as np
+
+    import bench
+    out = {"final_trans": torch.randn(5, 4, 4), "final_labels": torch.rand(5, 7)}
+    bench.dump_outputs(str(tmp_path / "all"), out, 0, 1)
+    assert sorted(os.listdir(tmp_path / "all")) == ["final_labels.npy", "final_trans.npy"]
+    for k, v in out.items():
+        a = np.load(tmp_path / "all" / f"{k}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, v.numpy())
+    B, N = 3000, 6000                                   # 72 MB of outputs
+    big = {"final_trans": torch.arange(B * 16, dtype=torch.float32).reshape(B, 4, 4), "final_labels": torch.zeros(B, N)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big, 0, 1)
+    sets = np.load(tmp_path / "a" / "sets.npy")
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 << 20
+    assert len(sets) > 2700 and np.array_equal(sets, np.load(tmp_path / "b" / "sets.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "final_trans.npy"), big["final_trans"].numpy()[sets.astype(np.int64)])
+
+
+@pytest.mark.gpu
+def test_bench_dumps_what_the_timed_steps_returned(tmp_path):
+    """The arrays `bench.py --dump-outputs` writes are what the module returns for the benchmark's seeded inputs."""
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    import bench
+    from pointdsc_b200 import PointDSC
+    subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--steps", "2", "--warmup", "1", "--n", "160", "--batch", "3",
+                    "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True,
+                   timeout=600, check=True)
+    model = PointDSC(in_dim=6, num_layers=12, num_channels=128, num_iterations=10, ratio=0.1, k=40, **bench.CTOR["3dmatch"])
+    model.load_state_dict(load_snapshot("3dmatch"), strict=False)
+    model = model.cuda().eval()
+    x = bench.make_inputs(160, 3, "3dmatch", 0)
+    want = model.run(*(x[k].cuda() for k in ("corr_pos", "src_keypts", "tgt_keypts")))
+    assert sorted(os.listdir(tmp_path)) == ["final_labels.npy", "final_trans.npy"]
+    for k in ("final_trans", "final_labels"):
+        assert np.array_equal(np.load(tmp_path / f"{k}.npy"), want[k].cpu().numpy()), k

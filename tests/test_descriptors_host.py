@@ -118,24 +118,16 @@ def test_oracle_fpfh_mass_and_rigid_invariance():
     assert np.median(diff) < 1e-4 and (diff < 2.0).mean() > 0.9, (np.median(diff), (diff < 2.0).mean())
 
 
-def _demo_clouds():
-    import os
-    from conftest import REPO
-    for root in (os.path.join(REPO, "baseline", "_ref", "demo_data"), "/root/reference/demo_data"):
-        paths = [os.path.join(root, f"cloud_bin_{i}.ply") for i in (0, 1)]
-        if all(os.path.exists(p) for p in paths):
-            return paths
-    return None
-
-
-def test_ply_reader_on_the_reference_demo_clouds():
-    """BASELINE.json configs[0] reads demo_data/cloud_bin_{0,1}.ply (binary little-endian float xyz, 258 342 / 268 977 vertices)."""
-    paths = _demo_clouds()
-    if paths is None:
-        pytest.skip("the reference's demo clouds are not installed (baseline/_ref/demo_data)")
+def test_ply_reader_on_the_reference_demo_clouds(tmp_path):
+    """BASELINE.json configs[0] reads demo_data/cloud_bin_{0,1}.ply (binary little-endian float xyz, 258 342 / 268 977 vertices,
+    CloudCompare's header): read here behind those same headers, with one vertex per 5 cm voxel of each cloud."""
+    from conftest import demo_clouds
+    paths, counts, points = demo_clouds(tmp_path)
+    assert counts == [258342, 268977]
     from pointdsc_b200.descriptors import read_ply
-    for path, n in zip(paths, (258342, 268977)):
+    for path, want in zip(paths, points):
+        n = len(want)
         pts = read_ply(path)
         assert pts.shape == (n, 3) and pts.dtype == np.float32 and np.isfinite(pts).all()
         raw = np.fromfile(path, dtype="<f4", offset=os.path.getsize(path) - 12 * n).reshape(n, 3)   # the payload behind the header
-        assert np.array_equal(pts, raw)
+        assert np.array_equal(pts, raw) and np.array_equal(pts, want)
